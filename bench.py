@@ -14,6 +14,9 @@ One JSON line on stdout (rank 0).  `value` = whole-job expl/s with inputs reside
 metric through the public API (LRP.generate_LRP_batched) with pinned-host inputs and a D2H read of the maps in
 every step; `roofline` = the dominant kernel (the z+ Linear-rule contraction) timed alone with CUDA events;
 `cpu_baseline` = the CPU oracle/reference timed on this box's host cores on a bounded sample.
+
+--dump-outputs DIR writes what the timed path returned in its last timed step (rank 0) as DIR/<name>.npy, float32 or
+float64: the inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -67,7 +70,32 @@ def parse():
                          "BASELINE batch as the GLOBAL batch, sharded over the GPUs (SURVEY 8e: 256 -> 32 per GPU at 8). "
                          "With N > 1 the weak run also reports the strong-scaling numbers under the key 'strong'.")
     ap.add_argument("--no-graph", action="store_true", help="strong-scaling line without CUDA-graph replay")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(path, arrays):
+    """Write each tensor of `arrays` (name -> tensor, leading dim = sample) as path/<name>.npy: floating outputs in
+    float32, integer ones (class indices) as float64.  When they exceed DUMP_LIMIT_BYTES together, the same fixed,
+    seeded sample of rows is taken from each and its row numbers are written as rows.npy."""
+    import numpy as np
+    arrays = {k: (v.float() if v.is_floating_point() else v.double()).detach().cpu() for k, v in arrays.items()}
+    n = next(iter(arrays.values())).shape[0]
+    row_bytes = sum(v[:1].numel() * v.element_size() for v in arrays.values())
+    if n * row_bytes > DUMP_LIMIT_BYTES:
+        keep = max(1, (DUMP_LIMIT_BYTES - 4096) // (row_bytes + 8))         # + 8 bytes per row of rows.npy, headers
+        rows = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:keep].sort().values
+        arrays = {k: v[rows] for k, v in arrays.items()}
+        arrays["rows"] = rows.double()
+    os.makedirs(path, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), v.numpy())
 
 
 def peaks():
@@ -411,9 +439,12 @@ def run_reference_arm(args, w):
             run(xs[i:i + 1]); i += 1
     t0 = time.perf_counter()
     for _ in range(args.steps):
+        maps = []
         for _ in range(per_step):
-            run(xs[i:i + 1]); i += 1
+            maps.append(run(xs[i:i + 1])); i += 1
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"maps": torch.cat(maps)})
     val = per_step * args.steps / dt
     sample = "%d B=1 explanations per step on %d host threads" % (per_step, torch.get_num_threads())
     line = {"impl": "reference", "metric": "explanations_per_sec", "value": round(val, 4), "unit": "expl/s",
@@ -466,11 +497,20 @@ def main():
     explain_call(w, eng, x_dev[:min(batch, 8)], min(batch, 8))       # allocator / module warm-up (untimed)
     torch.cuda.synchronize()
 
+    last = {}
+
+    def step():
+        last["out"] = explain_call(w, eng, x_dev, batch)
+
     sampler = ClockSampler(local)
     l0 = lib.te_kernel_launch_count()
     sampler.start()
-    ms = timed_steps(lambda: explain_call(w, eng, x_dev, batch), args.steps, args.warmup, world)
+    ms = timed_steps(step, args.steps, args.warmup, world)
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        maps, idx = last["out"]
+        dump_outputs(args.dump_outputs, {"maps": maps, "index": idx})
+    del last
     launches = (lib.te_kernel_launch_count() - l0) // max(1, (args.steps + args.warmup)) * args.steps
     value = world * batch * args.steps / (ms * 1e-3)
 

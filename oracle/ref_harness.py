@@ -3,8 +3,7 @@
 ``/root/reference`` does not exist on the GPU box; there the harness imports the
 byte-for-byte mirror of the hot-path files that ``oracle/fetch_ref.py`` leaves in
 ``oracle/_ref`` (git-ignored).  It is used by ``oracle/make_golden.py`` (fixture
-generation), by the ``-m "not gpu"`` tests that pin the oracle when the reference is
-present, and by ``bench.py``'s ``cpu_baseline`` leg / ``--impl reference`` arm.
+generation) and by ``bench.py``'s ``cpu_baseline`` leg / ``--impl reference`` arm.
 
 Shims (SURVEY.md §8c) — each one works around an incompatibility of the
 reference with this container, none changes the arithmetic:
