@@ -296,6 +296,33 @@ TE_API int te_f16_block_split(const float* x, int rows, int cols, void* hi, void
 TE_API int te_linear_backward_ex(const float* dy, const float* w, float* dx, float* scratch, int rows, int in_features,
                           int out_features, unsigned flags, void* stream);
 
+/* The attention-shaped contractions of the engines, through the engines' own dispatch — exported for kernel unit tests
+ * only.  A, B and X are head slices of packed activations [batch*n, ld] (head h at columns h*head_dim ..), addressed in
+ * place; rows of one sample follow those of the previous one.
+ *   te_attention_nn:  out[b,h,i,j] = epi(alpha * sum_d A[b*n+i, h*head_dim+d] * B[b*n+j, h*head_dim+d])
+ *     out and e are [batch, heads, n, ld_out] with ld_out >= round_up(n, 4).  epi: TE_ATTN_STORE, TE_ATTN_MUL (* e),
+ *     TE_ATTN_SD (safe_divide(e, .), layers_ours.py:10-13) or TE_ATTN_SOFTMAX (over j; e unused).
+ *   te_attention_nk:  out[b*n+m, h*head_dim+c] = epi(alpha * sum_k A_h[m,k] * X[b*n+k, h*head_dim+c])
+ *     A_h = map[b,h] (transpose = 0) or its transpose (transpose = 1); map is [batch, heads, n, np] (np >= n), X / out / e
+ *     are packed with row strides ldx / ld_out / ld_out.  epi: TE_ATTN_STORE or TE_ATTN_MUL.  The pad columns [n, np) of
+ *     map must hold finite values: the tensor-core kernel multiplies them by zero-filled operand rows, and NaN * 0 = NaN.
+ * flags: 0 runs the fp32 SIMT kernels; TE_FLAG_ATTN_TENSOR_CORES the tcgen05 3xTF32 kernels (te_set_option
+ * "attn_persistent" applies); | TE_FLAG_RELPROP_TF32 their single-pass TF32 form for STORE / MUL, which the N x N
+ * dispatch takes for n <= 256 only (beyond that it runs 3xTF32, as the engines do).  With the tensor-core flag a shape or
+ * epilogue the tcgen05 kernels do not take (head_dim other than 32 / 64, N x d at head_dim != 64, single-pass SD or
+ * SOFTMAX, row strides that are not multiples of 4) returns TE_ERR_UNSUPPORTED instead of running the SIMT kernel.
+ * SOFTMAX at n > 256 runs the tensor-core scores followed by the row-softmax kernel. */
+#define TE_ATTN_STORE 0
+#define TE_ATTN_MUL 1
+#define TE_ATTN_SD 2
+#define TE_ATTN_SOFTMAX 3
+TE_API int te_attention_nn(const float* a, int lda, const float* b, int ldb, int batch, int heads, int n,
+                           int head_dim, const float* e, float* out, int ld_out, float alpha, int epi, unsigned flags,
+                           void* stream);
+TE_API int te_attention_nk(const float* map, int np, int transpose, const float* x, int ldx, int batch, int heads, int n,
+                           int head_dim, const float* e, float* out, int ld_out, float alpha, int epi, unsigned flags,
+                           void* stream);
+
 #ifdef __cplusplus
 }
 #endif

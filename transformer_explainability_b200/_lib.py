@@ -105,7 +105,14 @@ PROTOTYPES = {
     "te_linear_forward_ex": (c_int, [_P, _P, _P, _P, _P, c_int, c_int, c_int, c_uint, _P]),
     "te_linear_backward_ex": (c_int, [_P, _P, _P, _P, c_int, c_int, c_int, c_uint, _P]),
     "te_f16_block_split": (c_int, [_P, c_int, c_int, _P, _P, _P, _P]),
+    "te_attention_nn": (c_int, [_P, c_int, _P, c_int, c_int, c_int, c_int, c_int, _P, _P, c_int, c_float, c_int, c_uint,
+                                _P]),
+    "te_attention_nk": (c_int, [_P, c_int, c_int, _P, c_int, c_int, c_int, c_int, c_int, _P, _P, c_int, c_float, c_int,
+                                c_uint, _P]),
 }
+
+# epilogues of te_attention_nn / te_attention_nk
+ATTN_STORE, ATTN_MUL, ATTN_SD, ATTN_SOFTMAX = 0, 1, 2, 3
 
 _lib = None
 

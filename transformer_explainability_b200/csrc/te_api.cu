@@ -9,6 +9,7 @@
 #include "te_rollout.h"
 #include "te_zplus.h"
 #include "te_gemm_tc.h"
+#include "te_engine_util.h"
 
 static thread_local std::string g_last_error;
 void te_set_last_error(const char* msg) { g_last_error = msg ? msg : ""; }
@@ -190,6 +191,62 @@ extern "C" int te_matmul_qk_relprop(const float* q, const float* k, const float*
     g.E0 = k; g.lde0 = d; g.sE1 = nd; g.M = n; g.N = d; g.K = n;
     TE_TRY(te_gemm_launch(g, TE_L_MN, TE_L_MN, TE_XF_NONE, TE_EPI_MUL, st));
     return TE_OK;
+}
+
+// ---- attention-shaped contractions through the engines' dispatch (te_engine_util.h), for kernel unit tests -------------
+static const unsigned kAttnFlags = TE_FLAG_ATTN_TENSOR_CORES | TE_FLAG_RELPROP_TF32;
+
+extern "C" int te_attention_nn(const float* a, int lda, const float* b, int ldb, int batch, int heads, int n, int head_dim,
+                               const float* e, float* out, int ld_out, float alpha, int epi, unsigned flags, void* stream) {
+    REQ(a && b && out && batch > 0 && heads > 0 && n > 0 && head_dim > 0, "te_attention_nn: bad argument");
+    REQ(epi >= TE_ATTN_STORE && epi <= TE_ATTN_SOFTMAX, "te_attention_nn: epi out of range");
+    REQ(e || epi == TE_ATTN_STORE || epi == TE_ATTN_SOFTMAX, "te_attention_nn: MUL / SD need e");
+    REQ(lda >= heads * head_dim && ldb >= heads * head_dim, "te_attention_nn: lda / ldb < heads * head_dim");
+    REQ(ld_out >= ((n + 3) & ~3), "te_attention_nn: ld_out < round_up(n, 4)");
+    REQ((long long)batch * heads <= 65535, "te_attention_nn: batch * heads > 65535");
+    REQ((flags & ~kAttnFlags) == 0 && (flags == 0 || (flags & TE_FLAG_ATTN_TENSOR_CORES)),
+        "te_attention_nn: flags other than TE_FLAG_ATTN_TENSOR_CORES [| TE_FLAG_RELPROP_TF32]");
+    const bool tc = (flags & TE_FLAG_ATTN_TENSOR_CORES) != 0, tf32 = (flags & TE_FLAG_RELPROP_TF32) != 0;
+    if (tc) {
+        // no SIMT stand-in for a shape the tcgen05 kernels do not take: a passing test must have run them
+        if (head_dim != 32 && head_dim != 64) { te_set_last_error("te_attention_nn: tcgen05 kernels take head_dim 32 / 64"); return TE_ERR_UNSUPPORTED; }
+        if (tf32 && epi != TE_ATTN_STORE && epi != TE_ATTN_MUL) {
+            te_set_last_error("te_attention_nn: the single-pass form has STORE / MUL epilogues only");
+            return TE_ERR_UNSUPPORTED;
+        }
+        if (!te_tc_attn_supported(n, head_dim, lda, ldb, ld_out)) {
+            te_set_last_error("te_attention_nn: shape / strides not supported by the tcgen05 kernel (or no driver)");
+            return TE_ERR_UNSUPPORTED;
+        }
+    }
+    cudaStream_t st = ST(stream);
+    if (epi == TE_ATTN_SOFTMAX) return te_util::attn_probs(tc, batch, heads, n, ld_out, head_dim, a, lda, b, ldb, out, alpha, st);
+    const int gepi = (epi == TE_ATTN_STORE) ? TE_EPI_STORE : (epi == TE_ATTN_MUL) ? TE_EPI_MUL : TE_EPI_SD;
+    return te_util::attn_nn(tc, batch, heads, n, ld_out, head_dim, a, lda, b, ldb, out, e, alpha, gepi, st, tf32);
+}
+
+extern "C" int te_attention_nk(const float* map, int np, int transpose, const float* x, int ldx, int batch, int heads, int n,
+                               int head_dim, const float* e, float* out, int ld_out, float alpha, int epi, unsigned flags,
+                               void* stream) {
+    REQ(map && x && out && batch > 0 && heads > 0 && n > 0 && head_dim > 0 && np >= n, "te_attention_nk: bad argument");
+    REQ(transpose == 0 || transpose == 1, "te_attention_nk: transpose is 0 or 1");
+    REQ(epi == TE_ATTN_STORE || epi == TE_ATTN_MUL, "te_attention_nk: epi out of range (STORE / MUL)");
+    REQ(e || epi == TE_ATTN_STORE, "te_attention_nk: MUL needs e");
+    REQ(ldx >= heads * head_dim, "te_attention_nk: ldx < heads * head_dim");
+    REQ(ld_out >= heads * head_dim, "te_attention_nk: ld_out < heads * head_dim");
+    REQ((long long)batch * heads <= 65535, "te_attention_nk: batch * heads > 65535");
+    REQ((flags & ~kAttnFlags) == 0 && (flags == 0 || (flags & TE_FLAG_ATTN_TENSOR_CORES)),
+        "te_attention_nk: flags other than TE_FLAG_ATTN_TENSOR_CORES [| TE_FLAG_RELPROP_TF32]");
+    const bool tc = (flags & TE_FLAG_ATTN_TENSOR_CORES) != 0, tf32 = (flags & TE_FLAG_RELPROP_TF32) != 0;
+    if (tc) {
+        if (head_dim != 64) { te_set_last_error("te_attention_nk: the tcgen05 kernel takes head_dim 64"); return TE_ERR_UNSUPPORTED; }
+        if (!te_tc_attn_nk_supported(n, head_dim, np, ldx, ld_out)) {
+            te_set_last_error("te_attention_nk: shape / strides not supported by the tcgen05 kernel (or no driver)");
+            return TE_ERR_UNSUPPORTED;
+        }
+    }
+    return te_util::attn_nk(tc, batch, heads, n, np, head_dim, map, transpose, x, ldx, out, ld_out, e, alpha,
+                            epi == TE_ATTN_STORE ? TE_EPI_STORE : TE_EPI_MUL, ST(stream), tf32);
 }
 
 static int g_cls_rows = 1;

@@ -138,6 +138,59 @@ def linear_backward_tf32(dy, w):
     return dx
 
 
+_ATTN_EPI = {"store": _lib.ATTN_STORE, "mul": _lib.ATTN_MUL, "sd": _lib.ATTN_SD, "softmax": _lib.ATTN_SOFTMAX}
+
+
+def _packed_rows(t, what):
+    """Row stride of a 2-D fp32 CUDA view with unit column stride (e.g. a column slice of a packed activation)."""
+    if t.dim() != 2 or t.dtype != torch.float32 or not t.is_cuda or t.stride(1) != 1:
+        raise ValueError("%s: 2-D fp32 CUDA view with unit column stride expected" % what)
+    return t.stride(0)
+
+
+@_on_device
+def attention_nn(a, b, batch, heads, epi="store", e=None, out=None, alpha=1.0, flags=0):
+    """TEST ONLY (kernel unit tests; the engines call the same dispatch internally).  The N x N attention contraction
+    ``out[b,h,i,j] = epi(alpha * sum_d a[b*n+i, h*dh+d] * b[b*n+j, h*dh+d])`` (see include/te_b200.h: te_attention_nn).
+    a, b: [batch*n, heads*dh] views with unit column stride (head slices of a packed qkv buffer, addressed in place);
+    out, e: contiguous [batch, heads, n, ld_out] (out allocated with ld_out = round_up(n, 4) when None);
+    epi: "store" | "mul" | "sd" | "softmax"; flags: 0 (fp32 SIMT) or FLAG_ATTN_TENSOR_CORES [| FLAG_RELPROP_TF32]."""
+    lda, ldb = _packed_rows(a, "attention_nn a"), _packed_rows(b, "attention_nn b")
+    if a.shape != b.shape or a.shape[0] % batch or a.shape[1] % heads:
+        raise ValueError("attention_nn: a, b [batch*n, heads*dh] expected")
+    n, dh = a.shape[0] // batch, a.shape[1] // heads
+    if out is None:
+        out = torch.empty(batch, heads, n, (n + 3) // 4 * 4, device=a.device, dtype=torch.float32)
+    _req(out, e)
+    if out.dim() != 4 or tuple(out.shape[:3]) != (batch, heads, n) or (e is not None and e.shape != out.shape):
+        raise ValueError("attention_nn: out / e [batch, heads, n, ld_out] expected")
+    check(_lib.load().te_attention_nn(ptr(a), lda, ptr(b), ldb, batch, heads, n, dh, ptr(e), ptr(out), out.shape[3], alpha,
+                                      _ATTN_EPI[epi], flags, _stream()), "te_attention_nn")
+    return out
+
+
+@_on_device
+def attention_nk(amap, x, heads, transpose=False, epi="store", e=None, out=None, alpha=1.0, flags=0):
+    """TEST ONLY (kernel unit tests; the engines call the same dispatch internally).  The token-reduced N x d contraction
+    ``out[b*n+m, h*dh+c] = epi(alpha * sum_k A_h[m,k] * x[b*n+k, h*dh+c])`` with A_h = amap[b,h] or its transpose
+    (see include/te_b200.h: te_attention_nk).  amap: contiguous [batch, heads, n, np] (pad columns finite);
+    x, out, e: [batch*n, heads*dh] views with unit column stride (out, e share one row stride; out allocated packed when
+    None); epi: "store" | "mul"; flags: 0 (fp32 SIMT) or FLAG_ATTN_TENSOR_CORES [| FLAG_RELPROP_TF32]."""
+    _req(amap)
+    ldx = _packed_rows(x, "attention_nk x")
+    if amap.dim() != 4 or amap.shape[1] != heads or x.shape[0] != amap.shape[0] * amap.shape[2] or x.shape[1] % heads:
+        raise ValueError("attention_nk: amap [batch, heads, n, np], x [batch*n, heads*dh] expected")
+    batch, n, np_ = amap.shape[0], amap.shape[2], amap.shape[3]
+    if out is None:
+        out = torch.empty(x.shape, device=x.device, dtype=torch.float32)
+    ld_out = _packed_rows(out, "attention_nk out")
+    if out.shape != x.shape or (e is not None and (e.shape != x.shape or _packed_rows(e, "attention_nk e") != ld_out)):
+        raise ValueError("attention_nk: out / e [batch*n, heads*dh] with one row stride expected")
+    check(_lib.load().te_attention_nk(ptr(amap), np_, int(transpose), ptr(x), ldx, batch, heads, n, x.shape[1] // heads,
+                                      ptr(e), ptr(out), ld_out, alpha, _ATTN_EPI[epi], flags, _stream()), "te_attention_nk")
+    return out
+
+
 @_on_device
 def linear_relprop(x, w, r, tensor_cores=False, y=None, bias=None, bf16=False, variant="ours", r_f16=False):
     """``Linear.relprop`` (layers_ours.py:207-230): x [...,in], w [out,in], r [...,out] -> [...,in].
